@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — preference-pairs/sec of one full LLaVA-1.5-7B DPO optimisation step on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W]            (N=1)
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--dump-outputs DIR]            (N=1)
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" = policy forward on chosen+rejected (CLIP -> projector -> splice -> 32 decoder layers ->
@@ -176,10 +176,12 @@ CHECKER_PARAM_SCALE = 0.3   # std multiplier of oracle.make_params for the full-
                             # orders agree to 5e-5 (tools/cpu_fullwidth_inherent.py)
 
 
-def full_width_case(num_layers, dtype=torch.float32):
-    """The oracle-side model / batch of the cpu_baseline leg: full width, config (a) shape (1 pair, R=64, T=687)."""
+def full_width_case(num_layers, dtype=torch.float32, cfg=None):
+    """The oracle-side model / batch of the cpu_baseline leg: full width (or `cfg`'s dims), config (a) shape (1 pair,
+    R=64, T=687)."""
+    import dataclasses
     from oracle import llava_dpo_oracle as O
-    cfg = O.OracleConfig(num_layers=num_layers)
+    cfg = O.OracleConfig(num_layers=num_layers) if cfg is None else dataclasses.replace(cfg, num_layers=num_layers)
     p = O.make_params(cfg, seed=0, dtype=dtype, scale=CHECKER_PARAM_SCALE)
     for k in p:
         if k.startswith(O.TRAINABLE_PREFIXES):
@@ -338,10 +340,10 @@ def _reference_step_fn(nl, cfg=None):
     return step
 
 
-def _port_step_fn(nl):
+def _port_step_fn(nl, cfg=None):
     """Fallback when oracle/_ref is not staged: the oracle port of the same path (kind "port")."""
     from oracle import llava_dpo_oracle as O
-    cfg, p, batch = full_width_case(nl, torch.float32)
+    cfg, p, batch = full_width_case(nl, torch.float32, cfg=cfg)
     names = O.trainable_names(p)
     state = {k: [torch.zeros_like(p[k]), torch.zeros_like(p[k])] for k in names}
 
@@ -434,8 +436,32 @@ def eva_flops_per_image(e, batch_tokens=None):
     return e.live_blocks * per_block + 2 * e.n_tokens * e.patch_k * C
 
 
-def run_workload(args, rank, local_rank, world, lora=False, omnilmm=False, steps=None, warmup=None, extras=False):
-    """One measured workload -> the JSON line (dict). `extras`: a reduced run used for the `extra` sub-records."""
+DUMP_SAMPLE = 1 << 21      # parameter / gradient entries --dump-outputs writes per store (8 MB per array in float32)
+
+
+def dump_outputs(out_dir, metrics, policy):
+    """`--dump-outputs DIR`: what the last timed step computed, as float32 .npy files — `metrics.npy`, the 9 values
+    train_step returned (engine.METRIC_NAMES order), and `params.npy` / `grads.npy`, the bf16 parameters after that
+    step's AdamW update and the gradients it produced, at DUMP_SAMPLE fixed, seeded positions of the flat store
+    (`lora_params.npy` / `lora_grads.npy` likewise for the adapters of a LoRA run)."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "metrics.npy"), metrics.float().cpu().numpy())
+    stores = [("", policy.store)]
+    if getattr(policy, "lora", None) is not None:
+        stores.append(("lora_", policy.lora))
+    for prefix, st in stores:
+        n = st.flat.numel()
+        g = torch.Generator().manual_seed(0)
+        idx = torch.randint(0, n, (min(DUMP_SAMPLE, n),), generator=g).sort().values.to(st.flat.device)
+        np.save(os.path.join(out_dir, prefix + "params.npy"), st.flat[idx].float().cpu().numpy())
+        np.save(os.path.join(out_dir, prefix + "grads.npy"), st.grad[idx].float().cpu().numpy())
+
+
+def run_workload(args, rank, local_rank, world, lora=False, omnilmm=False, steps=None, warmup=None, extras=False,
+                 dump_dir=None):
+    """One measured workload -> the JSON line (dict). `extras`: a run for one of the `extra` sub-records.
+    `dump_dir`: where rank 0 writes the outputs of the last timed step (dump_outputs)."""
     from rlaifv_b200 import lib, ops
     from rlaifv_b200.engine import DPOStepEngine
     from rlaifv_b200.model import LlavaDims, LlavaDPOPolicy
@@ -499,12 +525,14 @@ def run_workload(args, rank, local_rank, world, lora=False, omnilmm=False, steps
     loss_host = torch.zeros(9, dtype=torch.float32).pin_memory()
 
     def run_steps(batches, n, read_back):
+        m = None
         for s in range(n):
             m = engine.train_step(batches[s % len(batches)])
             if read_back:
                 loss_host.copy_(m, non_blocking=True)
                 torch.cuda.current_stream().synchronize()
         engine.opt.wait_all()      # the last step's parameter all-gathers belong to the timed region
+        return m
 
     try:
         step0 = engine.train_step(dev_batches[0], optimizer_step=False)   # known-answer check (no update)
@@ -532,12 +560,14 @@ def run_workload(args, rank, local_rank, world, lora=False, omnilmm=False, steps
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     t_host0 = time.perf_counter()
-    run_steps(dev_batches, steps, False)
+    last_metrics = run_steps(dev_batches, steps, False)
     host_enqueue_ms = (time.perf_counter() - t_host0) * 1e3 / steps   # CPU time to enqueue one step
     e1.record()
     barrier()
     ms_dev = e0.elapsed_time(e1) / steps
     launches = (lib.launch_count() - launches0) // max(1, steps)
+    if dump_dir and rank == 0:          # before the e2e steps below move the parameters on
+        dump_outputs(dump_dir, last_metrics, policy)
     # ---- end-to-end timing through the public call with host buffers (e2e) ----
     run_steps(host_batches, 1, True)
     barrier()
@@ -717,7 +747,12 @@ def main():
                          "(11.6 B trainable parameters: needs >= 2 GPUs for the ZeRO-2 sharded fp32 optimizer state)")
     ap.add_argument("--omnilmm-no-tower", action="store_true",
                     help="with --omnilmm: feed the tower's output tokens (the round-1 boundary; fits one GPU)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step as DIR/*.npy (see dump_outputs), so that two builds "
+                         "can be compared on the same seeded inputs")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
 
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -732,10 +767,10 @@ def main():
         os.environ.setdefault("MASTER_ADDR", "127.0.0.1")
         dist.init_process_group("nccl", device_id=torch.device("cuda", local_rank))
 
-    line = run_workload(args, rank, local_rank, world, lora=args.lora, omnilmm=args.omnilmm)
+    line = run_workload(args, rank, local_rank, world, lora=args.lora, omnilmm=args.omnilmm, dump_dir=args.dump_outputs)
     headline = not (args.lora or args.omnilmm)
     if headline and not args.no_extras:
-        # BASELINE configs (e) and (d) as driver-visible sub-records of the same run (short: 3 timed steps each).
+        # BASELINE configs (e) and (d) as sub-records of the same run, with the same --steps / --warmup.
         # Every rank runs them (collectives inside); a failure is recorded, never raised.
         extra = {}
         plan = [("lora_dpo_config_e", dict(lora=True, omnilmm=False))]
@@ -747,7 +782,7 @@ def main():
                                "fit one 180 GB GPU; measured at N >= 2 (ZeRO-2 shards the 139 GB optimizer state)"}
         for name, kw in plan:
             try:
-                sub = run_workload(args, rank, local_rank, world, steps=3, warmup=2, extras=True, **kw)
+                sub = run_workload(args, rank, local_rank, world, extras=True, **kw)
                 extra[name] = {k: sub[k] for k in EXTRA_KEYS if k in sub}
             except Exception as exc:                       # noqa: BLE001 - the headline line must survive
                 extra[name] = {"error": "%s: %s" % (type(exc).__name__, str(exc)[:300])}

@@ -53,12 +53,15 @@ def test_thread_calibration(bench_mod):
 
 def test_reference_arm_step_functions_run_at_tiny_dims(bench_mod):
     """Both step functions of the CPU arm (the staged unmodified reference, and the oracle-port fallback) complete an
-    optimisation step; the reference one only where oracle/_ref has been staged (build() does it in the build
-    container, the copy travels to the GPU box)."""
+    optimisation step; the reference one only where oracle/_ref has been staged (build() does it where the reference
+    tree is readable)."""
     from oracle import llava_dpo_oracle as O
     from oracle import stage_ref
+    makers = [bench_mod._port_step_fn]
     if stage_ref.available():
-        fn = bench_mod._reference_step_fn(2, cfg=O.TINY)
+        makers.append(bench_mod._reference_step_fn)
+    for make in makers:
+        fn = make(2, cfg=O.TINY)
         l0, l1 = fn(), fn()
         assert l0 == l0 and l1 == l1 and l0 != l1            # finite, and the AdamW step changed the model
         ts = bench_mod._time_cpu_steps(fn, 1, 2)
@@ -71,6 +74,31 @@ def test_reference_arm_other_ranks_exit_quietly():
     r = subprocess.run([sys.executable, os.path.join(REPO, "bench.py"), "--impl", "reference", "--gpus", "2"],
                        capture_output=True, text=True, env=env, timeout=300)
     assert r.returncode == 0 and r.stdout.strip() == ""
+
+
+def test_dump_outputs_writes_seeded_float32_samples(bench_mod, tmp_path):
+    """--dump-outputs: metrics plus parameter / gradient samples at the same seeded positions on every run, float32,
+    within 64 MB for a full-size LLaVA-1.5-7B LoRA run (two stores of four arrays)."""
+    import numpy as np
+    from types import SimpleNamespace
+    n = 3 * bench_mod.DUMP_SAMPLE
+
+    def store(off):
+        return SimpleNamespace(flat=torch.arange(n, dtype=torch.float32).to(torch.bfloat16),
+                               grad=torch.full((n,), off, dtype=torch.bfloat16))
+    policy = SimpleNamespace(store=store(1.0), lora=store(2.0))
+    metrics = torch.arange(9, dtype=torch.float32)
+    for d in ("a", "b"):
+        bench_mod.dump_outputs(str(tmp_path / d), metrics, policy)
+    names = sorted(os.listdir(tmp_path / "a"))
+    assert names == ["grads.npy", "lora_grads.npy", "lora_params.npy", "metrics.npy", "params.npy"]
+    for nm in names:
+        a, b = np.load(tmp_path / "a" / nm), np.load(tmp_path / "b" / nm)
+        assert a.dtype == np.float32 and np.array_equal(a, b)
+    assert np.array_equal(np.load(tmp_path / "a" / "metrics.npy"), metrics.numpy())
+    assert np.load(tmp_path / "a" / "params.npy").shape == (bench_mod.DUMP_SAMPLE,)
+    assert (np.load(tmp_path / "a" / "lora_grads.npy") == 2.0).all()
+    assert sum(os.path.getsize(tmp_path / "a" / nm) for nm in names) <= 64 * 2 ** 20
 
 
 def test_committed_bench_line_has_the_contract_keys():

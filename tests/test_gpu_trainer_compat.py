@@ -3,6 +3,7 @@ frozen-reference log-prob pre-pass vs oracle, train()/checkpoint/resume on a syn
 import os
 from types import SimpleNamespace
 
+import numpy as np
 import pytest
 import torch
 
@@ -183,39 +184,25 @@ def test_train_llava15_entry_end_to_end(tmp_path, monkeypatch):
     assert tuple(win["image"].shape) == (3, c.image_size, c.image_size) and win["image"].dtype == torch.float32
 
 
-def test_reference_compute_loss_text_on_rebound_seam(tmp_path):
-    """INTEGRATION.md §1, the two-line rebinding: the reference's OWN `LLaVA15DPOTrainer.compute_loss` source
-    (muffin/train/trainers.py:279-311, imported from the staged oracle/_ref copy) with only `get_beta_and_logps` and
-    `dpo_loss` rebound to this repo's, on the reference's own collator output. Loss / metrics must equal the fused
-    engine's on the same batch, and `loss.backward()` must drive the hand-written backward."""
-    from oracle import stage_ref
-    if not stage_ref.available():
-        pytest.skip("oracle/_ref not staged (build() stages it where /root/reference exists)")
-    stage_ref.import_reference()
-    import muffin.train.trainers as T
-    import rlaifv_b200.trainers as B
+SEAM_FIXTURE = os.path.join(os.path.dirname(__file__), "golden", "trainer", "compute_loss_seam.npz")
+
+
+def test_reference_compute_loss_text_on_rebound_seam():
+    """INTEGRATION.md §1, the two-line rebinding: the reference's OWN `LLaVA15DPOTrainer.compute_loss`
+    (muffin/train/trainers.py:279-311) with only `get_beta_and_logps` and `dpo_loss` rebound to this repo's, on the
+    collator output below. oracle/gen_golden_trainer_seam.py ran it on a B200 and stored its loss, the metrics it logs
+    and the gradient its `loss.backward()` drove through the hand-written backward (norm and a seeded sample). The
+    fused engine on the same batch must give the same loss, metrics and gradients."""
     from rlaifv_b200.collator import DataCollatorForDPODataset
     from rlaifv_b200.engine import DPOStepEngine
     from rlaifv_b200.llava_model import LlavaLlamaForCausalLM
+    fx = np.load(SEAM_FIXTURE)
     params = O.make_params(O.TINY, seed=0, scale=0.4)
-    model = LlavaLlamaForCausalLM(dims(), "cuda", hf_state=params)
+    assert abs(O.params_checksum(params) - float(fx["params_checksum"])) <= 1e-9 * float(fx["params_checksum"])
     batch = DataCollatorForDPODataset(tokenizer=Tok(), beta=0.1, mod_token_weight=1.0)(instances(2, seed=3))
-    saved = (T.get_beta_and_logps, T.dpo_loss)
-    T.get_beta_and_logps, T.dpo_loss = B.get_beta_and_logps, B.dpo_loss            # <- the rebinding
-    try:
-        logged = []
-        stub = SimpleNamespace(args=SimpleNamespace(past_index=-1, dpo_use_average=False, dpo_token_weighted=False,
-                                                    task="DPO"),
-                               _nested_gather=lambda x: x.reshape(1), log=logged.append)
-        model.policy.store.grad.zero_()
-        loss = T.LLaVA15DPOTrainer.compute_loss(stub, model, {k: (v.clone() if torch.is_tensor(v) else v)
-                                                              for k, v in batch.items()})
-        loss.backward()
-        model.policy.finalize_embed_grad()
-        torch.cuda.synchronize()
-    finally:
-        T.get_beta_and_logps, T.dpo_loss = saved
-    g_bridge = model.policy.store.grad.float().clone()
+    assert np.array_equal(batch["concatenated_input_ids"].numpy(), fx["concatenated_input_ids"])
+    assert np.array_equal(batch["concatenated_labels"].numpy(), fx["concatenated_labels"])
+    g_bridge = torch.from_numpy(fx["grad_sample"])
     assert float(g_bridge.abs().max()) > 0
     # the fused engine on the same batch (no optimizer step): same loss, same metrics, same gradients
     model2 = LlavaLlamaForCausalLM(dims(), "cuda", hf_state=params)
@@ -223,13 +210,14 @@ def test_reference_compute_loss_text_on_rebound_seam(tmp_path):
     m = eng.train_step(dict(batch), optimizer_step=False)
     md = eng.metrics_dict(m)
     torch.cuda.synchronize()
-    assert abs(float(loss) - md["loss"]) <= 1e-6 * max(1.0, abs(md["loss"]))
-    names = logged[0]
+    assert abs(float(fx["loss"]) - md["loss"]) <= 1e-6 * max(1.0, abs(md["loss"]))
     for k in ("rewards_train/chosen", "rewards_train/rejected", "rewards_train/accuracies", "rewards_train/margins",
               "logps_train/chosen", "logps_train/rejected", "logps_train/ref_chosen", "logps_train/ref_rejected"):
-        assert abs(names[k] - md[k]) <= 1e-5 * max(1.0, abs(md[k])), k
+        assert abs(float(fx["metric:" + k]) - md[k]) <= 1e-5 * max(1.0, abs(md[k])), k
     g_engine = model2.policy.store.grad.float()
-    assert float((g_bridge - g_engine).norm() / g_engine.norm()) <= 1e-3
+    sample = g_engine[torch.from_numpy(fx["grad_index"]).long().cuda()].cpu()
+    assert float((g_bridge - sample).norm() / sample.norm()) <= 1e-3
+    assert abs(float(fx["grad_norm"]) - float(g_engine.double().norm())) <= 1e-3 * float(g_engine.double().norm())
 
 
 def test_llava_token_weighted_extension_matches_spliced_oracle():
